@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU kernel on the host cores
+    python bench.py ... --dump-outputs DIR                   # + what the last timed step computed, as DIR/*.npy
 
 A "step" = one pass of the hot path (bin atoms -> scan -> scatter -> tile fill) over one batch of synthetic
 pockets: BASELINE.json configs[2] (256 protein pockets x ~3000 atoms, 64^3 grid @ 1 A, 8 channels) PER GPU
@@ -48,7 +49,15 @@ def parse():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the side measurements (C2 ligands, C5 fine grids, C4 distances)")
     ap.add_argument("--no-scaling", action="store_true", help="skip the strong-scaling / NCCL gather / config-4 section")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (rank 0) as DIR/<name>.npy, "
+                         "so that two builds can be compared output for output")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return a
 
 
 def make_workload(kind: str, batch: int, rank: int):
@@ -725,6 +734,27 @@ def scaling_section(a, dev, world, rank, peak):
     return out
 
 
+DUMP_ROWS = 1 << 20  # sampled grid rows: 1M rows x 8 channels x 4 B = 32 MB, the whole dump stays under 64 MB
+
+
+def dump_outputs(path, batch, out):
+    """Write what one step of the timed path returns, the float32 grid `out` (total_voxels, C), as .npy files under
+    `path`.  The grid of the flagship workload is GBs, so the files hold the rows at a fixed seeded sample of row indices,
+    in index order (occupancy_sample.npy, float32, (min(total_voxels, DUMP_ROWS), C)), and the float64 sum of every grid
+    and channel over the whole grid (occupancy_sum.npy, (B, C)).  The workloads are seeded, so the same arguments give
+    the same inputs."""
+    import torch
+
+    os.makedirs(path, exist_ok=True)
+    n = batch.total_voxels
+    rows = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_ROWS), replace=False))
+    np.save(os.path.join(path, "occupancy_sample.npy"), out[torch.from_numpy(rows).to(out.device)].cpu().numpy())
+    sums = np.zeros((batch.B, batch.C))
+    for b in range(batch.B):
+        sums[b] = out[int(batch.out_offsets[b]):int(batch.out_offsets[b + 1])].sum(dim=0, dtype=torch.float64).cpu().numpy()
+    np.save(os.path.join(path, "occupancy_sum.npy"), sums)
+
+
 def run_ours(a):
     import torch
     import torch.distributed as dist
@@ -776,6 +806,8 @@ def run_ours(a):
     t_wall1 = time.perf_counter()
     launches = _lib.launch_count(local) - l0
     ms_total = ev0.elapsed_time(ev1)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, batch, out)
     # per-kernel durations (one synchronising read per step, outside the aggregate timing above)
     for _ in range(a.steps):
         batch.run(d_coords, d_sig, out)

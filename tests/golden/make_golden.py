@@ -612,9 +612,26 @@ def xtc_fixture():
             os.remove(os.path.join(out_dir, fcache))
 
 
+def live_pins():
+    """live_reference.json: sha256 of the oracle's outputs on the seeded cases of the *_vs_live_reference tests of
+    tests/test_oracle_golden.py, so those comparisons also run where oracle/_ref is absent.  The tests record them
+    themselves (MKB_RECORD_LIVE=1); with oracle/_ref built they first assert that every output equals the reference
+    binary's, and the file notes per test whether that was the case."""
+    import subprocess
+
+    if os.path.isfile(os.path.join(HERE, "live_reference.json")):
+        os.remove(os.path.join(HERE, "live_reference.json"))
+    subprocess.run([sys.executable, "-m", "pytest", "-q", "-p", "no:cacheprovider",
+                    os.path.join(ROOT, "tests", "test_oracle_golden.py"), "-k", "live_reference or float_overloads"],
+                   check=True, cwd=ROOT, env=dict(os.environ, MKB_RECORD_LIVE="1"))
+
+
 def main():
     from oracle import build_ref
 
+    if "--only-live" in sys.argv:
+        live_pins()
+        return
     if "--only-xtc" in sys.argv:
         assert build_ref.build()
         xtc_fixture()

@@ -5,7 +5,9 @@ its compiled kernels taken from oracle/_ref (the reference's .pyx compiled by or
 read from the reference's test files, and the host prologues of ``MetricDistance.project`` / ``MetricSelfDistance`` -- string
 selections through ``mol.atomselect``, group building, ``digitize_chains``, the arguments that reach the kernel -- are
 compared with the reference's up to the kernel call (both kernels are replaced by recorders, nothing runs on a GPU).
-Skipped on the GPU box, where the reference tree does not exist.
+Where the reference tree does not exist, each test instead drives the same prologue from the reference's stored molecule
+fields and selection masks (tests/golden/traj20.npz), with the CPU oracle as the kernel, and compares the projection bit
+for bit with the reference's stored outputs of it: wrong selections, chain ids, groups, masses or flags change them.
 """
 import os
 import shutil
@@ -17,11 +19,13 @@ import pytest
 REF = "/root/reference"
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "moleculekit")), reason="reference tree not present")
 
 
 @pytest.fixture(scope="module")
 def refmol(tmp_path_factory):
+    """The reference's Molecule, or None where the reference tree is absent (the tests then use the stored data)."""
+    if not os.path.isdir(os.path.join(REF, "moleculekit")):
+        return None
     sys.path.insert(0, ROOT)
     from oracle import build_ref
 
@@ -82,12 +86,61 @@ def _capture_ours(monkeypatch, fn_name, build_and_project):
     return rec.calls[0]
 
 
+def _bits(a):
+    a = np.ascontiguousarray(a, dtype=np.float32)
+    b = a.view(np.uint32).copy()
+    b[np.isnan(a)] = 0x7FC00000
+    return b
+
+
+@pytest.fixture
+def stored_mol(g_traj, oracle, monkeypatch):
+    """The reference's molecule fields and selection masks as stored in traj20.npz, with the CPU oracle (the reference's
+    kernels restated in C) in place of the device kernels behind the projections."""
+    from moleculekit_b200 import distance_utils as du
+    from moleculekit_b200.molecule_lite import MolLite
+
+    def dist(coords, box, sel1, sel2, chains, selfdist, pbc, results, metric="distances", truncate=None, **kw):
+        assert metric == "distances" and truncate is None
+        oracle.dist_trajectory(coords, box, sel1, sel2, chains, selfdist, pbc, results)
+        return results
+
+    def reduction(coords, box, g1, g2, ch1, ch2, selfdist, pbc, masses, r1, r2, results, metric="distances", truncate=None,
+                  **kw):
+        assert metric == "distances" and truncate is None
+        oracle.dist_trajectory_reduction(coords, box, g1, g2, ch1, ch2, selfdist, pbc, masses, r1, r2, results)
+        return results
+
+    monkeypatch.setattr(du, "dist_trajectory", dist)
+    monkeypatch.setattr(du, "dist_trajectory_reduction", reduction)
+    g = g_traj
+    return MolLite(g["coords"], g["box"], element=g["element"], name=g["name"], resname=g["resname"], resid=g["resid"],
+                   chain=g["chain"], segid=g["segid"],
+                   named_selections={s: m for s, m in zip(g["sel_strings"].tolist(), g["sel_masks"])})
+
+
+# stored cases per `periodic`: selections, keyword arguments, the reference's stored projection output
+STORED_MD = {
+    None: ("protein and resid 1 to 50 and noh", "protein and resid 1 to 50 and noh",
+           dict(groupsel1="residue", groupsel2="residue"), "ref_selfmindistance"),
+    "chains": ("protein and resid 1 to 20 and noh", "resname MOL and noh", {}, "ref_chains_distances"),
+    "selections": ("protein and name CA", "resname MOL and noh", {}, "ref_distances"),
+}
+
+
 @pytest.mark.parametrize("periodic", [None, "chains", "selections"])
-def test_metricdistance_prologue_with_reference_molecule(refmol, monkeypatch, periodic):
+def test_metricdistance_prologue_with_reference_molecule(refmol, request, monkeypatch, periodic):
     """MetricDistance(string selections) on the reference Molecule: sel masks, chain ids, selfdist / pbc flags and the
     trajectory arrays that reach dist_trajectory are those of the reference (metricdistance.py:132-179, util.py:12-85)."""
-    from moleculekit.projections.metricdistance import MetricDistance as RefMD
     from moleculekit_b200.projections.metricdistance import MetricDistance as OurMD
+
+    if refmol is None:
+        mol, g = request.getfixturevalue("stored_mol"), request.getfixturevalue("g_traj")
+        sel1, sel2, kw, key = STORED_MD[periodic]
+        data = OurMD(sel1, sel2, periodic=periodic, metric="distances", **kw).project(mol)
+        assert data.shape == g[key].shape and np.array_equal(_bits(data), _bits(g[key]))
+        return
+    from moleculekit.projections.metricdistance import MetricDistance as RefMD
 
     sel1, sel2 = "protein and name CA and resid 10 to 40", "resname MOL and noh"
     ref_args = _capture_reference(monkeypatch, "dist_trajectory",
@@ -103,10 +156,18 @@ def test_metricdistance_prologue_with_reference_molecule(refmol, monkeypatch, pe
     assert ref_args[7].shape == our_args[7].shape and ref_args[7].dtype == our_args[7].dtype
 
 
-def test_selfdistance_and_mapping_with_reference_molecule(refmol, monkeypatch):
+def test_selfdistance_and_mapping_with_reference_molecule(refmol, request, monkeypatch):
     """MetricSelfDistance + groupsel="residue" + getMapping on the reference Molecule (metricdistance.py:244-364)."""
-    from moleculekit.projections.metricdistance import MetricSelfDistance as RefSD
     from moleculekit_b200.projections.metricdistance import MetricSelfDistance as OurSD
+
+    if refmol is None:
+        mol, g = request.getfixturevalue("stored_mol"), request.getfixturevalue("g_traj")
+        sel = "protein and resid 1 to 50 and noh"
+        data = OurSD(sel, periodic=None, groupsel="residue").project(mol)
+        assert np.array_equal(_bits(data), _bits(g["ref_selfmindistance"]))
+        assert len(OurSD(sel, periodic=None, groupsel="residue").getMapping(mol)) == g["ref_selfmindistance"].shape[1]
+        return
+    from moleculekit.projections.metricdistance import MetricSelfDistance as RefSD
 
     sel = "protein and name CA and resid 5 to 30"
     ref_args = _capture_reference(monkeypatch, "dist_trajectory", lambda: RefSD(sel, periodic=None).project(refmol))
@@ -123,10 +184,17 @@ def test_selfdistance_and_mapping_with_reference_molecule(refmol, monkeypatch):
     assert [list(np.atleast_1d(x)) for x in rm["atomIndexes"]] == [list(np.atleast_1d(x)) for x in om["atomIndexes"]]
 
 
-def test_reduction_prologue_with_reference_molecule(refmol, monkeypatch):
+def test_reduction_prologue_with_reference_molecule(refmol, request, monkeypatch):
     """Residue groups against a ligand (get_reduced_distances, util.py:88-223): groups, group chain ids, masses, flags."""
-    from moleculekit.projections.metricdistance import MetricDistance as RefMD
     from moleculekit_b200.projections.metricdistance import MetricDistance as OurMD
+
+    if refmol is None:
+        mol, g = request.getfixturevalue("stored_mol"), request.getfixturevalue("g_traj")
+        kw = dict(periodic="selections", groupsel1="residue", groupsel2="all")
+        data = OurMD("protein and noh", "resname MOL and noh", **kw).project(mol)
+        assert np.array_equal(_bits(data), _bits(g["ref_mindistances"]))
+        return
+    from moleculekit.projections.metricdistance import MetricDistance as RefMD
 
     kw = dict(periodic="selections", groupsel1="residue", groupsel2="all", metric="contacts", threshold=6)
     sel1, sel2 = "protein and resid 10 to 25 and noh", "resname MOL and noh"
