@@ -329,6 +329,32 @@ int mkb_ring_pairs_fill(mkb_handle_t h, void *stream, int32_t mode, const mkb_tr
                         const uint32_t *starts1, int64_t n_rings1, const uint32_t *second, int64_t n_second, float p0,
                         float p1, float p2, float p3, const int64_t *row_offsets, int32_t *pairs, float *distangles);
 
+/* K14: superposition of trajectory frames, replaces the frame loop of _pp_align / _pp_measure_fit (moleculekit/align.py,
+ * called from Molecule.align) and util.molRMSD.  frames [n_frames] int64 device: the frames of t to process (indexes into
+ * the view t, so a frame shard works as for K3); entry i of transforms / out belongs to frames[i].  sel [n_sel] uint32
+ * device; ref float32 device, row j of the selection, dim d, column c at ref[(j*3 + d)*ref_stride + c] (the selected rows,
+ * frame-minor like t->coords).  Index ranges are the caller's responsibility.
+ * fit  : transforms [n_frames][15] float64 device = R (3x3 row-major), cP, cQ: the proper rotation minimising
+ *        sum |(p - cP) R^T + cQ - q|^2 over the selection, p from frame frames[i] of t, q from reference column
+ *        matchingframes ? frames[i] : 0.  Centroids and covariance are summed in float64; the rotation is Horn's quaternion
+ *        (cyclic Jacobi on the 4x4 key matrix, float64).  It equals the reference's SVD with reflection correction wherever
+ *        that is unique (1e-12 relative, not bitwise), and is exactly the identity for a zero covariance (n_sel == 1,
+ *        coincident points), where the reference's SVD yields the identity too.
+ * apply: every atom of every listed frame of t->coords (MODIFIED IN PLACE): x' = (x - cP) R^T + cQ evaluated in float64
+ *        from the float32 input and rounded once to float32.  frames must not repeat.
+ * rmsd : out [n_frames] float32 device = sqrt(mean over the selection of |x' - r|^2), summed in float64, where x' is the
+ *        float32 value apply would store with transforms[i] (transforms == NULL: the stored coordinate) and r the reference
+ *        column ref_frames == 1 ? 0 : frames[i].
+ * No atomics: the fit and rmsd sums run in a fixed order that depends only on n_sel and min(32, pow2 >= n_frames), so
+ * identical calls return identical bits. */
+int mkb_align_fit(mkb_handle_t h, void *stream, const mkb_traj *t, const int64_t *frames, int64_t n_frames,
+                  const uint32_t *sel, int64_t n_sel, const float *ref, int64_t ref_stride, int32_t matchingframes,
+                  double *transforms);
+int mkb_align_apply(mkb_handle_t h, void *stream, const mkb_traj *t, const int64_t *frames, int64_t n_frames,
+                    const double *transforms);
+int mkb_rmsd(mkb_handle_t h, void *stream, const mkb_traj *t, const int64_t *frames, int64_t n_frames, const uint32_t *sel,
+             int64_t n_sel, const float *ref, int64_t ref_stride, int64_t ref_frames, const double *transforms, float *out);
+
 #ifdef __cplusplus
 }
 #endif

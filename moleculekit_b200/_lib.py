@@ -41,6 +41,7 @@ EXPORTS = [
     "mkb_cdist", "mkb_pdist", "mkb_squareform", "mkb_collisions_count", "mkb_collisions_fill",
     "mkb_bonds_count", "mkb_bonds_fill", "mkb_shell_counts", "mkb_wrap_box", "mkb_within_distance", "mkb_xtc_decode",
     "mkb_wrap_triclinic", "mkb_hbonds_count", "mkb_hbonds_fill", "mkb_ring_pairs_count", "mkb_ring_pairs_fill",
+    "mkb_align_fit", "mkb_align_apply", "mkb_rmsd",
 ]
 
 _lib = None
@@ -111,6 +112,9 @@ def load():
     lib.mkb_hbonds_fill.argtypes = [vp, vp, tp, vp, i64, vp, i64, vp, vp, f32, f32, i32, i32, vp, vp]
     lib.mkb_ring_pairs_count.argtypes = [vp, vp, i32, tp, vp, vp, i64, vp, i64, f32, f32, f32, f32, vp, C.POINTER(i64)]
     lib.mkb_ring_pairs_fill.argtypes = [vp, vp, i32, tp, vp, vp, i64, vp, i64, f32, f32, f32, f32, vp, vp, vp]
+    lib.mkb_align_fit.argtypes = [vp, vp, tp, vp, i64, vp, i64, vp, i64, i32, vp]
+    lib.mkb_align_apply.argtypes = [vp, vp, tp, vp, i64, vp]
+    lib.mkb_rmsd.argtypes = [vp, vp, tp, vp, i64, vp, i64, vp, i64, i64, vp, vp]
     for name in EXPORTS:
         if name in ("mkb_last_error", "mkb_launch_count", "mkb_version", "mkb_last_kernel", "mkb_occupancy_compact_blocks"):
             continue

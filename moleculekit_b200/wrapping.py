@@ -203,10 +203,11 @@ def getBondedGroups(mol, bonds=None):
     return np.hstack((grouplist, [n])).astype(np.uint32), grouparray
 
 
-def wrap(mol, wrapsel="all", fileBonds=True, guessBonds=False, wrapcenter=None, unitcell="rectangular", device=None):
-    """Mirror of Molecule.wrap (molecule.py:1987-2090); ``mol.coords`` is wrapped in place.  ``mol`` is duck-typed: coords,
-    box, numAtoms, bonds, atomselect (for a string ``wrapsel``), optionally boxangles / boxvectors and ``_getBonds``.
-    Cells with a box angle != 90 take the triclinic kernels with the reference's ``unitcell`` choice."""
+def wrap_plan(mol, wrapsel="all", fileBonds=True, guessBonds=False, wrapcenter=None, unitcell="rectangular"):
+    """Host bookkeeping of Molecule.wrap (molecule.py:1987-2090) without touching the coordinates: bonded groups, centre
+    selection or fixed centre, and the kernel choice.  Returns None when the reference skips the wrap (zero box), else a
+    dict with ``groups``, ``centersel``, ``center`` and ``unitcell`` (None = orthorhombic box, K9; else the triclinic
+    ``unitcell`` name, K9b, with ``boxvectors`` (3, 3, F) float64).  ``wrap`` and ``wrap_device`` both run on it."""
     unitcell = unitcell.lower()
     if unitcell not in ["rectangular", "triclinic", "compact"]:
         raise ValueError(f"Invalid unit cell type: {unitcell}. Must be one of: rectangular, triclinic, compact")
@@ -238,7 +239,7 @@ def wrap(mol, wrapsel="all", fileBonds=True, guessBonds=False, wrapcenter=None, 
             "Zero box size detected in `Molecule.box`; skipping wrap. "
             "Read a topology / trajectory containing box information, "
             "or set `mol.box` and `mol.boxangles` manually before calling `wrap`.")
-        return
+        return None
     if mol.box.shape[1] != mol.coords.shape[2]:
         raise RuntimeError(
             "Detected different number of simulation frames in `Molecule.box` and `Molecule.coords`. "
@@ -251,16 +252,49 @@ def wrap(mol, wrapsel="all", fileBonds=True, guessBonds=False, wrapcenter=None, 
             from .bondguesser import guess_bonds
             bonds = np.vstack((bonds, guess_bonds(mol))).astype(np.uint32)
     groups, _ = getBondedGroups(mol, bonds)
+    plan = {"groups": groups, "centersel": centersel, "center": wrapcenter, "unitcell": None, "boxvectors": None}
     boxangles = getattr(mol, "boxangles", None)
     if boxangles is None or not np.any(np.asarray(boxangles) != 90):  # molecule.py:2075-2077
-        wrap_box(groups, mol.coords, mol.box, centersel, wrapcenter, device=device)
-        return
+        return plan
     boxvectors = getattr(mol, "boxvectors", None)
     if boxvectors is None:
         boxvectors = box_vectors(mol.box, boxangles)
-    boxvectors = np.ascontiguousarray(boxvectors, dtype=np.float64)
-    if unitcell == "triclinic":
-        wrap_triclinic_unitcell(groups, mol.coords, boxvectors, centersel, wrapcenter, device=device)
+    plan["unitcell"] = unitcell
+    plan["boxvectors"] = np.ascontiguousarray(boxvectors, dtype=np.float64)
+    return plan
+
+
+def wrap(mol, wrapsel="all", fileBonds=True, guessBonds=False, wrapcenter=None, unitcell="rectangular", device=None):
+    """Mirror of Molecule.wrap (molecule.py:1987-2090); ``mol.coords`` is wrapped in place.  ``mol`` is duck-typed: coords,
+    box, numAtoms, bonds, atomselect (for a string ``wrapsel``), optionally boxangles / boxvectors and ``_getBonds``.
+    Cells with a box angle != 90 take the triclinic kernels with the reference's ``unitcell`` choice."""
+    plan = wrap_plan(mol, wrapsel, fileBonds, guessBonds, wrapcenter, unitcell)
+    if plan is None:
+        return
+    groups, centersel, wrapcenter = plan["groups"], plan["centersel"], plan["center"]
+    if plan["unitcell"] is None:
+        wrap_box(groups, mol.coords, mol.box, centersel, wrapcenter, device=device)
+    elif plan["unitcell"] == "triclinic":
+        wrap_triclinic_unitcell(groups, mol.coords, plan["boxvectors"], centersel, wrapcenter, device=device)
     else:
-        wrap_compact_unitcell(groups, mol.coords, boxvectors, centersel, wrapcenter, 1 if unitcell == "compact" else 0,
-                              device=device)
+        wrap_compact_unitcell(groups, mol.coords, plan["boxvectors"], centersel, wrapcenter,
+                              1 if plan["unitcell"] == "compact" else 0, device=device)
+
+
+def wrap_device(coords: torch.Tensor, box, plan) -> torch.Tensor:
+    """Runs a ``wrap_plan`` on a resident (N, 3, F) float32 trajectory in place (K9 / K9b) and returns it; ``box`` is the
+    host (3, F) box of the plan's molecule.  The same index checks as the host entry points run before the device call."""
+    if plan is None or coords.shape[0] == 0 or coords.shape[2] == 0:
+        return coords
+    groups, centersel = plan["groups"], plan["centersel"]
+    _check_index_ranges(groups, centersel, coords.shape[0])
+    dev = coords.device
+    d_groups = torch.from_numpy(np.ascontiguousarray(groups).view(np.int32)).to(dev)
+    d_cs = torch.from_numpy(np.ascontiguousarray(centersel).view(np.int32)).to(dev) if centersel.size else None
+    if plan["unitcell"] is None:
+        if groups.shape[0] < 2:
+            return coords
+        d_box = torch.from_numpy(np.ascontiguousarray(box, dtype=np.float32)).to(dev)
+        return wrap_box_device(coords, d_box, d_groups, d_cs, plan["center"])
+    d_bv = torch.from_numpy(plan["boxvectors"]).to(dev)
+    return wrap_triclinic_device(coords, d_bv, d_groups, d_cs, plan["center"], plan["unitcell"])
